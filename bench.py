@@ -1,13 +1,19 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the DSPi hot path on B200 (contract: see DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One *step* = one pass of the 10-band EQ cascade over one batch: 65 536 channels x 6144 samples
 (= 64 firmware packets of 96 frames @96 kHz) per GPU, channel-major float32, in place.
 N>1 is launched by torchrun, one rank per GPU; channels shard with no data-path collective
 (weak scaling: 65 536 channels per GPU, 524 288 at N=8 = BASELINE config 5).
 Rank 0 prints ONE JSON line.
+
+--dump-outputs DIR writes what the last timed step left in its buffer as DIR/eq_out.npy, so that two builds
+can be compared output for output: the rows of a fixed, seeded sample of channels (every frame), float32, or
+float64 for the int32 Q28 words (exact).  Inputs and parameters come from fixed seeds, so the same arguments
+give the same inputs on every run.  With N>1 GPUs only rank 0 writes, so the sample is drawn from rank 0's channel
+shard (the first channels of the job); the other shards are not in the file.
 """
 import argparse
 import json
@@ -25,6 +31,20 @@ METRIC = "audio samples/sec (whole box) at 65536ch x 10-band EQ, 96 kHz; % HBM r
 CHANNELS_PER_GPU = 65536
 FS = 96000.0
 ALG_BYTES_PER_SAMPLE = 8          # 4 B read + 4 B written per channel-sample (SURVEY.md §8d)
+DUMP_BYTES = 32 << 20             # --dump-outputs: size of the channel sample written
+
+
+def dump_outputs(out_dir, buf, q28):
+    """DIR/eq_out.npy: rows of ``buf`` (a [C][T] device tensor) for a sample of channels drawn with a fixed seed,
+    as many as fit DUMP_BYTES (at least one)."""
+    import torch
+    Cn, T = buf.shape
+    dtype = np.float64 if q28 else np.float32
+    n = max(1, min(Cn, DUMP_BYTES // (T * np.dtype(dtype).itemsize)))
+    rows = np.sort(np.random.default_rng(0).choice(Cn, n, replace=False))
+    y = buf[torch.from_numpy(rows).to(buf.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "eq_out.npy"), y.astype(dtype))
 
 
 def measured_peak_gbs():
@@ -271,7 +291,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output (a channel sample; with N>1 GPUs, of rank 0's shard only) to DIR/eq_out.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "dspi_b200":
+        ap.error("--dump-outputs applies to the GPU path (--impl dspi_b200)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -344,6 +369,8 @@ def main():
     clocks = sampler.stop()
     ms = ev0.elapsed_time(ev1)
     launches = eng.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, bufs[(args.steps - 1) % nbuf], q)
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -19,3 +19,10 @@ def test_reference_arm_line():
     assert line["cpu_baseline"]["kind"] in ("reference", "port") and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0 and line["gpu_launches"] == 0
     assert "workload" in line["config"] and "model" not in line["config"]
+
+
+def test_rejected_arguments(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and "error" in out.stderr, (extra, out.stderr[-500:])
+    assert not any(tmp_path.iterdir())
